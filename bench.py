@@ -23,10 +23,15 @@ roofline / cpu_baseline : see DESIGN.md "Measurement".
 
 --impl reference : the CPU port of the reference path (oracle/torch_cpu.py, all host cores) on the same
          workload - TensorFlow itself is not installable here (SURVEY.md 8c).
+
+--dump-outputs DIR : after the timed pass, write what the last timed microbatch (W+K-1) returned to its caller,
+         DIR/probs.npy (float32, G*B x 1000), so that two builds can be compared output for output on the same
+         seeded weights and inputs.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import queue
@@ -38,6 +43,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True     # the tree may be read-only: the bench writes nothing into it
 
 import numpy as np  # noqa: E402
 
@@ -64,7 +70,27 @@ def parse_args():
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--batch1-roofline", action="store_true",
                     help="also time every op on a single-image microbatch (the un-coalesced launch)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step to DIR/probs.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "b200":
+            ap.error("--dump-outputs applies to --impl b200")
+        os.makedirs(args.dump_outputs, exist_ok=True)
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, probs):
+    """Write the arrays the timed path returned; a larger output keeps every k-th row so the file stays within
+    DUMP_LIMIT_BYTES."""
+    probs = np.ascontiguousarray(probs, np.float32)
+    stride = -(-probs.nbytes // DUMP_LIMIT_BYTES)
+    np.save(Path(out_dir) / "probs.npy", probs[::stride])
 
 
 # engine defaults (measured on B200, profiles/README.md round 2): G queue items per launch, lanes per stage
@@ -102,6 +128,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-lms", "50", "-i", str(self.gpu_index)],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.terminate)    # an error before stop() must not leave the sampler running
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -252,7 +279,7 @@ def workload_config(args):
 # ----------------------------------------------------------------------------------------------- B200 arm
 def run_b200(args):
     from defer_b200 import _cabi
-    _cabi.load()                      # before torch initialises CUDA (sets CUDA_DEVICE_MAX_CONNECTIONS)
+    _cabi.load(build_if_missing=False)   # before torch initialises CUDA (sets CUDA_DEVICE_MAX_CONNECTIONS)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -404,22 +431,28 @@ def run_b200(args):
         r.mark_after(m1, 1)
     barrier_sync()
 
-    def direct_pass(n, start):
-        """Issue n microbatches back to back, limited only by back-pressure (at most max_inflight in flight)."""
+    def direct_pass(n, start, keep=None):
+        """Issue n microbatches back to back, limited only by back-pressure (at most max_inflight in flight).
+        One process: returns a copy of microbatch `keep`'s output (None if not asked for)."""
         if ctx is None:
             last_st = my_stages[-1]
             inflight = 0
             out = np.empty(last_st.out_shape, np.float32)
+            kept = None
             for s in range(start, start + n):
                 if inflight == depth:
                     last_st.result(s - depth, out)
+                    if s - depth == keep:
+                        kept = out.copy()
                     inflight -= 1
                 for r in my_stages:
                     r.step(s)
                 inflight += 1
             for s in range(start + n - inflight, start + n):
                 last_st.result(s, out)
-            return
+                if s == keep:
+                    kept = out.copy()
+            return kept
         # one process per GPU: rank 0 steps stage 0 and publishes `submitted`; node loops follow
         if rank == 0:
             for s in range(start, start + n):
@@ -444,9 +477,14 @@ def run_b200(args):
                 time.sleep(50e-6)
         threading.Thread(target=drain, daemon=True).start()
     tw0 = time.perf_counter()
-    direct_pass(total, seq0)
+    last_out = direct_pass(total, seq0, keep=m1 if args.dump_outputs else None)
     tw1 = time.perf_counter()
     windows.append((tw0, tw1))
+    if args.dump_outputs and rank == 0:
+        if ctx is not None:
+            # the last rank published every result into the ring; the T < ring tail rows have not overwritten m1's
+            last_out = ctx.results[m1 % ctx.ring].reshape(EB, -1)
+        dump_outputs(args.dump_outputs, last_out)
     ms = max(r.mark_elapsed_ms() for r in my_stages)
     barrier_sync()
     if ctx is not None and rank == 0:

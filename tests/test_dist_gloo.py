@@ -52,8 +52,9 @@ class FakeRunner:
 
 def _worker(rank, world, port, q):
     sys.path.insert(0, str(ROOT))
+    # host-only test: with a GPU visible DistContext would bind rank r to cuda:r, which a one-GPU machine lacks
     os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), MASTER_ADDR="127.0.0.1",
-                      MASTER_PORT=str(port))
+                      MASTER_PORT=str(port), CUDA_VISIBLE_DEVICES="")
     import threading
     from defer_b200.dist import DistContext
     from defer_b200.node import Node
@@ -184,8 +185,9 @@ class _HostStage:
 
 def _worker_defer(rank, world, port, q):
     sys.path.insert(0, str(ROOT))
+    # host-only test: with a GPU visible DistContext would bind rank r to cuda:r, which a one-GPU machine lacks
     os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), MASTER_ADDR="127.0.0.1",
-                      MASTER_PORT=str(port))
+                      MASTER_PORT=str(port), CUDA_VISIBLE_DEVICES="")
     import queue as pyqueue
     import threading
     import defer_b200.node as node_mod

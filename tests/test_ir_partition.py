@@ -34,7 +34,8 @@ def test_get_previous_single_and_list(resnet50):
     assert dag_util.get_previous(resnet50, "add_1") == ["bn2b_branch2c", "activation_3"]
 
 
-def test_construct_model_layer_sets_match_reference_rule(resnet50):
+def test_construct_model_layer_sets_match_reference_rule():
+    resnet50 = applications.ResNet50()     # not the shared fixture: other tests partition that one too
     cuts = applications.RESNET50_TEST_CUTS
     d = DEFER(list(range(8)))
     parts = d._partition(resnet50, cuts)
